@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- FasterSeg student (arch_1, F12.L16) inference FPS @ 1x3x1024x2048 on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one 1024x2048 frame through the student network (BASELINE.json configs[1]).
@@ -20,6 +20,8 @@ One "step" = one 1024x2048 frame through the student network (BASELINE.json conf
   cpu_baseline: the CPU oracle port of the reference path (same weights) on the host cores (N=1, rank 0 only)
 Multi-GPU: inference has no exchange step -> N independent replicas ("replicas only"), weak scaling.
 `--impl reference` times the reference's CPU path (oracle port; the Python reference tree does not exist on the GPU box).
+`--dump-outputs DIR`: after the timed steps, DIR/logits.npy holds what the last one computed (see dump_outputs); weights and input
+frames are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -382,6 +384,21 @@ def run_reference(args):
     print(json.dumps(line))
 
 
+DUMP_PIXELS = 1 << 19
+DUMP_SEED = 2024
+
+
+def dump_outputs(directory, logits):
+    """The frame's NCHW logits as float32 DIR/logits.npy of shape (N, C, DUMP_PIXELS): every class at DUMP_PIXELS pixel positions
+    drawn without replacement from a fixed seed and kept in row-major order (40 MB instead of the 159 MB of the full frame)."""
+    import numpy as np
+    n, c, h, w = logits.shape
+    pix = np.sort(np.random.RandomState(DUMP_SEED).choice(h * w, min(DUMP_PIXELS, h * w), replace=False))
+    sample = logits.reshape(n, c, h * w).index_select(2, torch.from_numpy(pix).to(logits.device))
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "logits.npy"), sample.float().cpu().numpy())
+
+
 def frame_sigma_roofline(model, x, frame_us):
     """Whole-frame efficiency: sum over the frame's launches of max(FLOPs / tensor peak, algorithmic bytes / HBM peak) at the
     measured peaks, divided by the measured frame time (SURVEY section 8d).  The launch list comes from one eager forward
@@ -541,10 +558,14 @@ def main():
     ap.add_argument("--no-supernet-step", action="store_true",
                     help="skip the secondary metrics (supernet pretrain / search step, BASELINE configs[2] / [4]; distillation "
                          "step, configs[3])")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the logits the last one computed to DIR/logits.npy (a fixed sample of pixels)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
-        if args.steps > 30:
-            args.steps = 30  # bounded CPU sample (a frame costs ~0.2-1 s of CPU time)
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes what our timed path computed; it has no meaning with --impl reference")
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
 
@@ -587,10 +608,12 @@ def main():
     st, en = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     st.record()
     for i in range(args.steps):
-        runner(pool[i % npool])
+        logits = runner(pool[i % npool])
     en.record()
     torch.cuda.synchronize()
     ms_total = st.elapsed_time(en)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, logits)
     if world > 1:
         t = torch.tensor([ms_total], device=device)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -311,21 +311,3 @@ def test_normalisation_table_matches_the_reference_normalize(name):
     assert abs(float(frame.astype(np.float64).sum()) - want["sum"]) <= 1e-6 * max(1.0, abs(want["sum"]))
     np.testing.assert_allclose(frame.reshape(-1)[:12], np.array(want["first"], dtype=np.float32), rtol=0, atol=0)
     np.testing.assert_allclose(frame.reshape(-1)[-12:], np.array(want["last"], dtype=np.float32), rtol=0, atol=0)
-
-
-def test_metric_goldens_are_what_the_live_reference_computes():
-    from oracle import make_golden_metric as mk
-    from oracle import ref_harness
-    if not ref_harness.reference_available():
-        pytest.skip("reference tree not mounted")
-    metric, normalize = mk.reference_modules()
-    gold = H.load_json("metric.json")
-    for name in mk.CASES:
-        n_cl, pred, gt = mk.metric_inputs(name)
-        hist, labeled, correct = metric.hist_info(n_cl, pred, gt)
-        assert hist.tolist() == gold["metric"][name]["hist"] and int(labeled) == gold["metric"][name]["labeled"]
-        assert int(correct) == gold["metric"][name]["correct"]
-    for name in mk.NORMALIZE_CASES:
-        img, mean, std = mk.normalize_inputs(name)
-        got = np.stack([normalize(im, mean, std) for im in img]).astype(np.float32)
-        assert got.reshape(-1)[:12].tolist() == gold["normalize"][name]["first"]

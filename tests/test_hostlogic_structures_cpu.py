@@ -1,118 +1,65 @@
 """Wiring of the derived network for structures the shipped genotypes do not exercise -- three branches, a branch that ends
 at 1/8 (its feature is copied straight into the fusion buffer), single-branch networks, eval and train builds -- on random
-architectures: the UNMODIFIED reference network (CPU fp32, imported from the mounted reference tree) and ours (CPU stand-in
-backend) get the same state_dict and the same input.  Random genotypes with random weights are badly conditioned (zoomed
-operators on 4x8 feature maps: the reference's own logits move by up to 30 % when it is merely run in torch fp16), so the
-gate is two-sided: our deviation from the fp32 reference must not exceed 1.5 x the deviation of the reference run in fp16
--- a mis-wired branch or concat offset produces O(1) errors and is far outside that band for the well-conditioned cases.
-Skipped where the reference tree is not mounted."""
-import copy
-
+architectures: ours (CPU stand-in backend) against the UNMODIFIED reference network (CPU fp32) given the same state_dict and the
+same input, through goldens (oracle/make_golden_fuzz.py, tests/golden/fuzz_forward.npz: the reference's outputs at fixed
+sample positions, its full argmax map).  Random genotypes with random weights are badly conditioned (zoomed operators on 4x8
+feature maps: the reference's own logits move by several % when it is merely run in torch fp16), so the gate is two-sided: our
+deviation from the fp32 reference must not exceed 1.5 x the deviation of the reference run in fp16 -- a mis-wired branch or
+concat offset produces O(1) errors and is far outside that band for the well-conditioned cases."""
+import numpy as np
 import pytest
 import torch
-import torch.nn as nn
 
 from oracle import make_golden_decode as mk
-from oracle import ref_harness
+from oracle import make_golden_fuzz as fz
 from tests import cpu_backend
-
-pytestmark = pytest.mark.skipif(not ref_harness.reference_available(), reason="reference tree not mounted")
-
-CASES = [(1003, [0, 1, 2]), (1010, [2, 0]), (1017, [1]), (1024, [0]), (1031, [1, 0]), (1038, [2]), (1045, [2, 1])]
-
-
-def _build(Net, case, lasts):
-    alphas, betas, ratios = mk.clone_params(case)
-    m = Net(alphas, betas, ratios, num_classes=19, layers=case["layers"], Fch=12, width_mult_list=mk.WML,
-            stem_head_width=case["stem_head_width"], ignore_skip=case["ignore_skip"])
-    m.eval()
-    m.build_structure(list(lasts))
-    return m
+from tests import helpers as H
 
 
 @pytest.fixture(scope="module")
-def reference_net():
-    return ref_harness.load_reference("train", "model_seg").model_seg.Network_Multi_Path_Infer
+def golden():
+    return H.load_npz("fuzz_forward.npz")
 
 
-@pytest.mark.parametrize("seed,lasts", CASES)
-def test_eval_logits_match_the_reference_on_random_structures(reference_net, seed, lasts):
+@pytest.mark.parametrize("seed,lasts", fz.EVAL_CASES)
+def test_eval_logits_match_the_reference_on_random_structures(golden, seed, lasts):
     from fasterseg_b200.model_seg import Network_Multi_Path_Infer
-    case = mk.draw_case(seed)
-    ref = _build(reference_net, case, lasts)
-    torch.manual_seed(seed)
-    with torch.no_grad():
-        for mod in ref.modules():      # variance-preserving conv init (torch's default shrinks the signal into fp16 subnormals
-            if isinstance(mod, nn.Conv2d):   # over 40 layers) and non-trivial BatchNorm statistics / affine, like a trained net
-                nn.init.kaiming_normal_(mod.weight, mode="fan_in", nonlinearity="relu")
-            if isinstance(mod, nn.BatchNorm2d):
-                mod.running_mean.normal_(0, 0.1)
-                mod.running_var.uniform_(0.5, 1.5)
-                mod.weight.normal_(1.0, 0.1)
-                mod.bias.normal_(0, 0.1)
-    ours = _build(Network_Multi_Path_Infer, case, lasts)
-    assert list(ours.state_dict()) == list(ref.state_dict())
-    ours.load_state_dict(ref.state_dict())
-    x = torch.randn(1, 3, 128, 256)
-    with torch.no_grad():
-        want = ref(x)
-        half = copy.deepcopy(ref).half()(x.half()).float()      # the reference itself, fp16 end to end (torch CPU kernels)
-        with cpu_backend.installed():
-            got = ours(x)
-            labels = ours.predict_labels(x)
-    assert got.shape == want.shape == (1, 19, 128, 256)
-    err = float((got - want).norm() / want.norm())
-    err16 = float((half - want).norm() / want.norm())
-    print("seed %d lasts %s layers %d: norm-wise rel err ours %.3e | reference in fp16 %.3e" % (seed, lasts, case["layers"], err, err16))
+    cid = fz.case_id("eval", seed, lasts)
+    ours = fz.build_derived(Network_Multi_Path_Infer, mk.draw_case(seed), lasts, False)
+    assert fz.keys_digest(list(ours.state_dict())) == str(golden[cid + "/keys"])
+    fz.init_weights(ours, seed)
+    x = fz.input_frame(seed, 1)
+    with torch.no_grad(), cpu_backend.installed():
+        got = ours(x)
+        labels = ours.predict_labels(x)
+    assert tuple(got.shape) == tuple(golden[cid + ".0/shape"]) == (1, 19, 128, 256)
+    err = fz.rel_err(fz.sample(got), golden[cid + ".0/want"].astype(np.float64))
+    err16 = float(golden[cid + ".0/err16"])
+    print("seed %d lasts %s: norm-wise rel err ours %.3e | reference in fp16 %.3e" % (seed, lasts, err, err16))
     assert err <= 1.5 * err16 + 2e-3
-    agree = float((labels.long() == want.argmax(1)).float().mean())
-    agree16 = float((half.argmax(1) == want.argmax(1)).float().mean())
-    assert agree >= agree16 - 0.02
+    agree = float((labels.long().numpy() == golden[cid + "/argmax"]).mean())
+    assert agree >= float(golden[cid + "/agree16"]) - 0.02
 
 
-@pytest.mark.parametrize("seed,lasts", [(1003, [0, 1, 2]), (1010, [2, 0]), (1017, [1]), (1045, [2, 1]), (1052, [1, 2])])
-def test_train_mode_auxiliary_heads_match_the_reference_on_random_structures(reference_net, seed, lasts):
+@pytest.mark.parametrize("seed,lasts", fz.TRAIN_CASES)
+def test_train_mode_auxiliary_heads_match_the_reference_on_random_structures(golden, seed, lasts):
     """Train-mode build (auxiliary 1/16 and 1/32 heads, model_seg.py:217-226,298-335) for `lasts` combinations the shipped
     genotypes do not cover: which features feed heads16 / heads32, in which order, and which predictions are None."""
     from fasterseg_b200.model_seg import Network_Multi_Path_Infer
-
-    def build(Net):
-        alphas, betas, ratios = mk.clone_params(case)
-        m = Net(alphas, betas, ratios, num_classes=19, layers=case["layers"], Fch=12, width_mult_list=mk.WML,
-                stem_head_width=case["stem_head_width"], ignore_skip=case["ignore_skip"])
-        m.train()
-        m.build_structure(list(lasts))
-        return m
-
-    case = mk.draw_case(seed)
-    ref = build(reference_net)
-    torch.manual_seed(seed)
-    with torch.no_grad():
-        for mod in ref.modules():
-            if isinstance(mod, nn.Conv2d):
-                nn.init.kaiming_normal_(mod.weight, mode="fan_in", nonlinearity="relu")
-            if isinstance(mod, nn.BatchNorm2d):
-                mod.weight.normal_(1.0, 0.1)
-                mod.bias.normal_(0, 0.1)
-    ours = build(Network_Multi_Path_Infer)
-    assert list(ours.state_dict()) == list(ref.state_dict())
-    ours.load_state_dict(ref.state_dict())
-    x = torch.randn(2, 3, 128, 256)
-    with torch.no_grad():
-        want = ref(x)
-        half = copy.deepcopy(ref)
-        half.load_state_dict(ours.state_dict())        # running stats as before the reference's forward touched them
-        half = half.half()
-        got16 = half(x.half())
-        with cpu_backend.installed():
-            got = ours(x)
-    assert len(got) == len(want) == 3
-    for name, g, w, h in zip(("pred8", "pred16", "pred32"), got, want, got16):
-        assert (g is None) == (w is None), name
-        if w is None:
+    cid = fz.case_id("train", seed, lasts)
+    ours = fz.build_derived(Network_Multi_Path_Infer, mk.draw_case(seed), lasts, True)
+    assert fz.keys_digest(list(ours.state_dict())) == str(golden[cid + "/keys"])
+    fz.init_weights(ours, seed)
+    x = fz.input_frame(seed, 2)
+    with torch.no_grad(), cpu_backend.installed():
+        got = ours(x)
+    assert len(got) == len(golden[cid + "/none"]) == 3
+    for i, (name, g) in enumerate(zip(("pred8", "pred16", "pred32"), got)):
+        assert (g is None) == bool(golden[cid + "/none"][i]), name
+        if g is None:
             continue
-        assert g.shape == w.shape
-        err = float((g.float() - w).norm() / w.norm())
-        err16 = float((h.float() - w).norm() / w.norm())
+        assert tuple(g.shape) == tuple(golden["%s.%d/shape" % (cid, i)])
+        err = fz.rel_err(fz.sample(g), golden["%s.%d/want" % (cid, i)].astype(np.float64))
+        err16 = float(golden["%s.%d/err16" % (cid, i)])
         print("seed %d lasts %s %s: ours %.3e | reference in fp16 %.3e" % (seed, lasts, name, err, err16))
         assert err <= 1.5 * err16 + 5e-3, name

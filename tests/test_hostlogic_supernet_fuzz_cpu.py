@@ -1,62 +1,36 @@
 """Supernet wiring with RANDOM architecture parameters (the goldens use the constant 1e-3 initialisation): MixedOp weights,
 beta mixing of the two cell invocations, width selection in every mode incl. gumbel-sampled `arch_ratio`, for several
-depths -- the UNMODIFIED reference (CPU fp32) against ours on the CPU stand-in backend, same state_dict, same RNG seeds,
-two-sided gate against the reference run in torch fp16 (random supernets are ill-conditioned, see
-tests/test_hostlogic_structures_cpu.py).  Skipped where the reference tree is not mounted."""
-import copy
-
+depths -- ours on the CPU stand-in backend against the UNMODIFIED reference (CPU fp32) given the same state_dict and the same
+RNG seeds, through goldens (oracle/make_golden_fuzz.py, tests/golden/fuzz_forward.npz), with a two-sided gate against the
+reference run in torch fp16 (random supernets are ill-conditioned, see tests/test_hostlogic_structures_cpu.py)."""
 import numpy as np
 import pytest
-import torch
-import torch.nn as nn
 
+from oracle import make_golden_fuzz as fz
 from oracle import make_golden_latency as mkl
-from oracle import ref_harness
 from tests import cpu_backend
-
-pytestmark = pytest.mark.skipif(not ref_harness.reference_available(), reason="reference tree not mounted")
+from tests import helpers as H
 
 
 @pytest.fixture(scope="module")
-def reference_supernet():
-    return ref_harness.load_reference("search", "slimmable_ops", "operations", "seg_oprs", "genotypes", "model_search").model_search.Network_Multi_Path
+def golden():
+    return H.load_npz("fuzz_forward.npz")
 
 
-@pytest.mark.parametrize("layers,arch_idx,mode,seed", [(5, 0, "max", 1), (5, 1, None, 2), (6, 1, "min", 3), (8, 1, None, 4), (8, 0, "random", 5)])
-def test_eval_forward_matches_reference_with_random_arch_parameters(reference_supernet, layers, arch_idx, mode, seed):
+@pytest.mark.parametrize("layers,arch_idx,mode,seed", fz.SUPERNET_CASES)
+def test_eval_forward_matches_reference_with_random_arch_parameters(golden, layers, arch_idx, mode, seed):
     from fasterseg_b200.model_search import Network_Multi_Path
-    ref = mkl.build(reference_supernet, layers).eval()
-    mkl.randomise_arch(ref, 900 + seed)
-    torch.manual_seed(seed)
-    with torch.no_grad():
-        for mod in ref.modules():
-            if isinstance(mod, nn.Conv2d):
-                nn.init.kaiming_normal_(mod.weight, mode="fan_in", nonlinearity="relu")
-            if isinstance(mod, nn.BatchNorm2d) and mod.running_mean is not None:
-                mod.running_mean.normal_(0, 0.1)
-                mod.running_var.uniform_(0.5, 1.5)
-                mod.weight.normal_(1.0, 0.1)
-                mod.bias.normal_(0, 0.1)
+    cid = fz.case_id("supernet", layers, arch_idx, mode, seed)
     ours = mkl.build(Network_Multi_Path, layers).eval()
-    assert [k for k, _ in ours.named_parameters()] == [k for k, _ in ref.named_parameters()]
-    ours.load_state_dict(ref.state_dict())
-    half = copy.deepcopy(ref).half()
-    x = torch.randn(1, 3, 128, 256)
-
-    def run(model, inp):
-        model.arch_idx, model.prun_mode = arch_idx, mode
-        np.random.seed(seed)          # 'random' widths
-        torch.manual_seed(100 + seed)  # gumbel noise of 'arch_ratio'
-        with torch.no_grad():
-            return model(inp)
-
-    want = run(ref, x)
-    got16 = run(half, x.half())
+    assert fz.keys_digest([k for k, _ in ours.named_parameters()]) == str(golden[cid + "/keys"])
+    mkl.randomise_arch(ours, 900 + seed)
+    fz.init_weights(ours, seed)
     with cpu_backend.installed():
-        got = run(ours, x)
-    assert len(got) == len(want) == 5
-    for i, (g, w, h) in enumerate(zip(got, want, got16)):
-        err = float((g - w).norm() / w.norm())
-        err16 = float((h.float() - w).norm() / w.norm())
+        got = fz.run_supernet(ours, fz.input_frame(seed, 1), arch_idx, mode, seed)
+    assert len(got) == 5
+    for i, g in enumerate(got):
+        assert tuple(g.shape) == tuple(golden["%s.%d/shape" % (cid, i)])
+        err = fz.rel_err(fz.sample(g), golden["%s.%d/want" % (cid, i)].astype(np.float64))
+        err16 = float(golden["%s.%d/err16" % (cid, i)])
         print("layers %d arch %d mode %s pred%d: ours %.3e | reference in fp16 %.3e" % (layers, arch_idx, mode, i, err, err16))
         assert err <= 1.5 * err16 + 3e-3, i

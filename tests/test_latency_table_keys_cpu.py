@@ -1,18 +1,13 @@
 """N3 preparation: the key space enumerated by tools/build_latency_table.py is exactly the key set of the reference's
-shipped lookup table (skipped where the reference tree is not mounted), and every key parses into one of our operators."""
-import os
-
-import numpy as np
+shipped lookup table (stored in tests/golden/latency_lookup_table.json), and every key parses into one of our operators."""
 import pytest
 
+from tests import helpers as H
 from tools import build_latency_table as blt
 
-REF_TABLE = "/root/reference/train/latency_lookup_table.npy"
 
-
-@pytest.mark.skipif(not os.path.isfile(REF_TABLE), reason="reference tree not mounted")
 def test_enumerated_keys_equal_the_reference_table():
-    ref = set(np.load(REF_TABLE, allow_pickle=True).item())
+    ref = set(H.load_json("latency_lookup_table.json"))
     ours = blt.table_keys()
     assert len(ours) == len(set(ours))
     assert set(ours) == ref, (sorted(ref - set(ours))[:5], sorted(set(ours) - ref)[:5])
